@@ -62,7 +62,16 @@ def parse():
     ap.add_argument("--profile-step", action="store_true",
                     help="run warm-up + the timed steps inside an NVTX range 'atlas_b200_timed' and exit (for ncu "
                          "--nvtx --nvtx-include 'atlas_b200_timed/'; no JSON line is printed)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float32 / "
+                         "float64, at most 64 MB): the same arguments give the same inputs, so two builds can be "
+                         "compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
 
 
 def peaks(kind="hbm"):
@@ -527,6 +536,41 @@ def gpu_reference_leg(args, bank, dev, steps=3, warmup=1):
     return out
 
 
+DUMP_LOGITS_BYTES = 48 << 20     # --dump-outputs: the logits in full up to this size, else a fixed sample of their rows
+DUMP_ENC_ROWS = 2048             # ... and a fixed sample of the encoder-state rows (6 MB), 64 MB in all
+
+
+def _sample_rows(t, n, seed):
+    """`t` [rows, width] -> (t[rows], rows): a fixed seeded sample of `n` rows in ascending order."""
+    import torch
+
+    rows = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(seed))[:n].sort().values
+    return t[rows.to(t.device)], rows
+
+
+def dump_outputs(out_dir, out, gids, scores):
+    """--dump-outputs: what one timed step returned, as out_dir/<name>.npy - the FiD loss and logits, a row sample of
+    the encoder states, and the retrieved global passage ids (float64, exact) with their scores.  16-bit values are
+    widened to float32."""
+    import numpy as np
+
+    loss, logits, enc = out
+    arrays = {"loss": loss.float(), "passage_ids": gids.double(), "passage_scores": scores.float()}
+    flat = logits.reshape(-1, logits.shape[-1])
+    keep = DUMP_LOGITS_BYTES // (flat.shape[1] * 4)
+    if flat.shape[0] <= keep:
+        arrays["logits"] = logits.float()
+    else:                           # the *_rows arrays index the rows of the tensor flattened to [-1, last dimension]
+        sample, rows = _sample_rows(flat, keep, 1)
+        arrays["logits_sample"], arrays["logits_sample_rows"] = sample.float(), rows.double()
+    enc = enc.reshape(-1, enc.shape[-1])
+    sample, rows = _sample_rows(enc, min(DUMP_ENC_ROWS, enc.shape[0]), 2)
+    arrays["encoder_states_sample"], arrays["encoder_states_sample_rows"] = sample.float(), rows.double()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.cpu().numpy())
+
+
 def run_ours(args):
     import ctypes
 
@@ -605,7 +649,7 @@ def run_ours(args):
             tok = bank_tokens.splice(gids, TEXT_LEN, rq_ids, rq_lens)
             out = reader(input_ids=tok["input_ids"].view(B, -1), attention_mask=tok["attention_mask"].view(B, -1),
                          decoder_input_ids=dec, labels=labels)
-        return out[0], gids, scores
+        return out, gids, scores
 
     def step_api():
         """The same step through the module surface train.py / evaluate.py call, HOST inputs and outputs: query strings
@@ -642,10 +686,15 @@ def run_ours(args):
         torch.cuda.nvtx.range_push("atlas_b200_timed")
         e0.record()
         for _ in range(args.steps):
-            loss, gids, _ = step_device()
+            last = None             # drop the previous step's logits / encoder states before the next step allocates
+            last = step_device()
         e1.record()
         barrier_sync()
         torch.cuda.nvtx.range_pop()
+    loss = last[0][0]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last)
+    del last
     if args.profile_step:
         if world > 1:
             dist.destroy_process_group()

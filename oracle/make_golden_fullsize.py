@@ -3,9 +3,10 @@ CPU (oracle/ref_shims.py) at the BASELINE shapes (VERDICT r1 "next round" item 1
 
   fid_base_full         `src.fid.FiD`, T5-v1.1-base dims (12 + 12 layers, d 768, 12 heads, d_ff 2048, vocab 32128), ONE query x
                         n_context 40 x text_maxlength 384 tokens (ragged passage lengths), 32 target tokens: fp32 logits
-                        (a strided column sample: every 8th vocabulary entry + the 64 largest of every row), loss, a row
+                        (a strided column sample: every 32nd vocabulary entry + the 64 largest of every row), loss, a row
                         sample of the encoder states - and the SAME quantities with the reference's parameters cast to bf16
-                        (how far the reference itself drifts at 16 bits = the accuracy budget of the GPU test).
+                        (how far the reference itself drifts at 16 bits = the accuracy budget of the GPU test).  The
+                        samples keep the file under 1 MB; the 16-bit runs are stored as float16 (checked lossless).
   contriever_base_full  `src.retrievers.Contriever`, BERT-base dims, 64 passages x <= 192 tokens: fp32 embeddings + the
                         reference's own bf16 run.
   untied_tiny           `src.retrievers.UntiedDualEncoderRetriever` (src/retrievers.py:108-135) with
@@ -44,7 +45,7 @@ def contriever_base_inputs(B=64):
 
 def logit_sample(logits):
     """[B, T, V] -> (strided columns, top-64 indices per row from the fp32 run are chosen by the caller)."""
-    return logits[..., ::8]
+    return logits[..., ::32]
 
 
 def fid_base():
@@ -78,7 +79,7 @@ def fid_base():
         out[f"logits_top_{name}"] = torch.gather(logits, -1, top_idx).numpy()
         out[f"argmax_{name}"] = logits.argmax(-1).numpy().astype(np.int32)
         enc = res.encoder_last_hidden_state.float()[0]
-        out[f"enc_rows_{name}"] = enc[::61].numpy()                           # 252 of the 15 360 rows
+        out[f"enc_rows_{name}"] = enc[::122].numpy()                          # 126 of the 15 360 rows
         out[f"enc_absmax_{name}"] = np.array(float(enc.abs().max()))
         print(f"fid_base {name}: {time.time() - t0:.1f} s, loss {float(res[0]):.5f}", flush=True)
     for k in ("logits_strided", "logits_top", "enc_rows"):
@@ -86,6 +87,9 @@ def fid_base():
             d = np.abs(out[f"{k}_{h16}"] - out[k + "_fp32"])
             print(f"  reference {h16} vs fp32 {k}: max abs diff {d.max():.4e}, mean {d.mean():.4e}, "
                   f"scale {np.abs(out[k + '_fp32']).max():.3f}")
+            half = out[f"{k}_{h16}"].astype(np.float16)
+            assert np.array_equal(half.astype(np.float32), out[f"{k}_{h16}"]), f"{k}_{h16} is not float16-exact"
+            out[f"{k}_{h16}"] = half
     np.savez_compressed(os.path.join(GOLDEN_DIR, "fid_base_full.npz"), weights_sha256=sha, **out)
 
 

@@ -19,12 +19,10 @@ DIM = 768
 
 
 def reference_root():
-    """Where the reference sources are importable from: the staged copy first (GPU box), else the mounted reference."""
+    """Where the reference sources are importable from: the copy oracle/make_ref.py staged inside the tree, or None."""
     staged = os.path.join(HERE, "_ref")
     if os.path.isfile(os.path.join(staged, "src", "index.py")):
         return staged
-    if os.path.isfile("/root/reference/src/index.py"):
-        return "/root/reference"
     return None
 
 

@@ -53,16 +53,15 @@ def _make_cpu_index_class():
     return OracleBackedIndex
 
 
-def _worker(rank, world, name, port, tmpdir, store_mode, capacity=None):
+def _worker(rank, world, name, rendezvous, tmpdir, store_mode, capacity=None):
     sys.path.insert(0, ROOT)
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     import synth
     import mips_oracle
 
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world),
-                      ATLAS_B200_PASSAGE_STORE=store_mode)
-    torch.distributed.init_process_group("gloo", rank=rank, world_size=world)
+    os.environ.update(RANK=str(rank), WORLD_SIZE=str(world), ATLAS_B200_PASSAGE_STORE=store_mode)
+    torch.distributed.init_process_group("gloo", init_method=f"file://{rendezvous}", rank=rank, world_size=world)
     try:
         g = load_golden(name)
         bank, q, nq_per_rank = golden_inputs(g)
@@ -115,9 +114,9 @@ def _worker(rank, world, name, port, tmpdir, store_mode, capacity=None):
                                                        ("w2_grid", 2, "exchange", None),
                                                        ("w4_grid_empty_rank", 4, "shm", 64), ("w2_grid", 2, "shm", 64)])
 def test_search_knn_host_logic_gloo(name, world, store, capacity):
-    port = 29710 + world + (7 if store == "exchange" else 0) + (11 if capacity else 0)
-    with tempfile.TemporaryDirectory() as tmp:
-        mp.spawn(_worker, args=(world, name, port, tmp, store, capacity), nprocs=world, join=True)
+    # rendezvous through a file of a private directory: no fixed TCP port that a concurrent run on the same host could hold
+    with tempfile.TemporaryDirectory() as tmp, tempfile.TemporaryDirectory() as rdzv:
+        mp.spawn(_worker, args=(world, name, os.path.join(rdzv, "store"), tmp, store, capacity), nprocs=world, join=True)
 
 
 def test_capacity_overflow_raises():

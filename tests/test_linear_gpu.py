@@ -144,7 +144,7 @@ def test_fused_rmsnorm_around_the_gemm(dev, dtype, M):
     (20780, 1032, 520, 1),      # M = 40 x 512 + 300: ... partly out of range; ragged N and K
     (16384, 4096, 768, 4),      # gated-GELU epilogue
 ])
-def test_quad_cluster_multicast_tiles(dev, dtype, M, N, K, epi):
+def test_quad_cluster_multicast_tiles(dev, dtype, M, N, K, epi, tmp_path):
     """Shapes large enough for the 4-CTA-cluster kernel (two CTA pairs sharing the W tile through TMA multicast): against the
     fp32 reference, and bit-identical to the 2-CTA pair kernel (same MMA order per output element: the accumulation over K
     is the same sequence of UMMA K = 16 steps in both)."""
@@ -176,9 +176,8 @@ def test_quad_cluster_multicast_tiles(dev, dtype, M, N, K, epi):
         "y = ops.linear(x, w, bias if epi in (1, 2, 3) else None, res if epi == 3 else None, epilogue=epi)\n"
         "torch.save(y.cpu(), sys.argv[1])\n"
     ) % (os.path.dirname(os.path.dirname(os.path.abspath(__file__))), M, N, K, epi, str(dtype).split(".")[1])
-    path = f"/tmp/_pair_{M}_{N}_{K}_{epi}_{str(dtype).split('.')[1]}.pt"
+    path = str(tmp_path / "quad.pt")
     env = dict(os.environ, ATLAS_B200_GEMM_QUAD="1")     # the child runs the opt-in quad-cluster kernel
     subprocess.run([sys.executable, "-c", code, path], check=True, env=env, timeout=300)
-    y_pair = torch.load(path)
-    os.remove(path)
-    assert torch.equal(y.cpu(), y_pair), "the quad-cluster kernel and the pair kernel disagree"
+    y_quad = torch.load(path)
+    assert torch.equal(y.cpu(), y_quad), "the quad-cluster kernel and the pair kernel disagree"
